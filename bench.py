@@ -2,6 +2,7 @@
 """bench.py -- headline benchmark of the MSM / NTT hot paths.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--lg-msm 26] [--lg-ntt 24]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one BLS12-381 G1 MSM over 2^26 synthetic points (BASELINE.json's headline metric),
@@ -11,7 +12,9 @@ through the drop-in C-ABI `mult_pippenger` with HOST (pinned) buffers (at N > 1:
 shard through `mult_pippenger`, then the same all-gather + combine).  The Goldilocks 2^24 NTT
 (the metric's second half) is measured in the same run and reported under "ntt".
 Timing: CUDA events on the launching stream, barrier + synchronize on both sides, max over
-ranks.  Inputs (8.6 GB MSM, 2 x 128 MiB NTT + L2 flush) exceed the 126 MB L2.
+ranks.  Inputs (8.6 GB MSM, 2 x 128 MiB NTT + L2 flush) exceed the 126 MB L2.  Every timed
+loop of every leg runs exactly --steps iterations; the untimed warm-up runs --warmup of them
+(at least 3 for the NTT and Pallas legs, whose first calls build tables and pools).
 """
 import argparse
 import ctypes as C
@@ -216,7 +219,13 @@ def main():
     ap.add_argument("--skip-cpu", action="store_true")
     ap.add_argument("--skip-ref-gpu", action="store_true")
     ap.add_argument("--lg-pallas", type=int, default=24)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step of each leg returned to DIR/<name>.npy "
+                         "(float64, every value exact; see dump_outputs).  With one rank: the BLS12-381 and Pallas "
+                         "MSMs and the Goldilocks NTT; with several ranks: the two MSMs only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -303,7 +312,7 @@ def main():
     # ---- roofline leg: the dominant kernel (bucket accumulation), timed live with CUDA events
     _lib.profile_enable(True)
     acc_ms = []
-    for _ in range(2):
+    for _ in range(args.steps):
         msm.msm_dev(msm.BLS12_381_G1, d_points, d_scalars)
         phases = dict(_lib.profile_read())
         acc_ms.append(phases.get("accumulate", 0.0))
@@ -347,9 +356,9 @@ def main():
         torch.cuda.empty_cache()
         msm.multi_scalar_mult(pts_host, sc_host)                        # warm the pools
         t0 = time.perf_counter()
-        for _ in range(max(1, args.steps)):
+        for _ in range(args.steps):
             r2 = msm.multi_scalar_mult(pts_host, sc_host)
-        dt = (time.perf_counter() - t0) / max(1, args.steps)
+        dt = (time.perf_counter() - t0) / args.steps
         e2e = {"value": 1.0 / dt, "unit": "MSM/s", "h2d_bytes_per_step": int(n * 128),
                "d2h_bytes_per_step": 144, "ms_per_step": dt * 1e3, "api": "mult_pippenger (host pointers, pinned)",
                "same_result": bool(_jac_equal(r2, result, msm))}
@@ -387,10 +396,10 @@ def main():
         e2e_step()                                                   # warm the pools
         barrier()
         t0 = time.perf_counter()
-        for _ in range(max(1, args.steps)):
+        for _ in range(args.steps):
             r2 = e2e_step()
         barrier()
-        dt = max_over_ranks((time.perf_counter() - t0) * 1e3 / max(1, args.steps)) * 1e-3
+        dt = max_over_ranks((time.perf_counter() - t0) * 1e3 / args.steps) * 1e-3
         bad = max_over_ranks(0.0 if failed is None else 1.0)        # agreed on by all ranks
         if bad == 0.0:
             e2e = {"value": 1.0 / dt, "unit": "MSM/s", "h2d_bytes_per_step": int(n_total * 128),
@@ -404,11 +413,13 @@ def main():
         e2e = {"value": None, "unit": "MSM/s", "h2d_bytes_per_step": int(n * 128), "d2h_bytes_per_step": 144,
                "note": "--skip-e2e"}
 
+    outputs = {"msm_bls12_381_affine": affine_words(result, P_BLS, 6)}
+
     # ---------------------------------------------------------------- Goldilocks NTT (second half of the metric)
-    ntt_res = bench_ntt(args, torch, ntt, _lib, peak, peak_src, barrier, max_over_ranks, world)
+    ntt_res = bench_ntt(args, torch, ntt, _lib, peak, peak_src, barrier, max_over_ranks, world, outputs)
 
     # ---------------------------------------------------------------- config 4: Pallas MSM, sharded like the headline
-    pallas = bench_pallas(args, torch, msm, parallel, barrier, max_over_ranks, rank, world)
+    pallas = bench_pallas(args, torch, msm, parallel, barrier, max_over_ranks, rank, world, outputs)
 
     # ---------------------------------------------------------------- the reference's own sm_100a kernels (N = 1)
     ref_gpu = None
@@ -439,6 +450,8 @@ def main():
                 "clocks": clocks, "e2e": e2e, "gpu_launches": int(gpu_launches), "roofline": roofline,
                 "cpu_baseline": cpu, "check": check, "ntt": ntt_res, "pallas_msm": pallas,
                 "reference_gpu": ref_gpu}
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
         emit(line)
     if world > 1:
         dist.destroy_process_group()
@@ -472,10 +485,52 @@ def _jac_equal(a, b, msm, field=0, nl=6):
     return np.array_equal(mul(a[nl:2 * nl], mul(zb2, zb)), mul(b[nl:2 * nl], mul(za2, za)))
 
 
+P_BLS = 0x1a0111ea397fe69a4b1ba7b6434bacd764774b84f38512bf6730d2a0f6b0f6241eabfffeb153ffffb9feffffffffaaab
+P_PALLAS = 0x40000000000000000000000000000000224698fc094cf91b992d30ed00000001   # base field of Pallas
+NTT_DUMP_SAMPLE = 1 << 20        # Goldilocks NTT positions written by --dump-outputs
+
+
+def words32(a):
+    """uint64 array (..., k) -> (..., 2k) float64 of its little-endian 32-bit words (exact)."""
+    a = np.ascontiguousarray(a, dtype=np.uint64)
+    return a.view(np.uint32).reshape(*a.shape[:-1], 2 * a.shape[-1]).astype(np.float64)
+
+
+def affine_words(jac, p, nl):
+    """Jacobian point of the library (X, Y, Z Montgomery residues, nl 64-bit limbs each) -> the
+    affine x = X/Z^2, y = Y/Z^3 as plain integers, (2, 2*nl) float64 32-bit words; the point at
+    infinity is all zeros.  Unlike the Jacobian coordinates, which depend on the order the
+    buckets were summed in, this is the same for every computation of the same group element."""
+    jac = np.asarray(jac, dtype=np.uint64)
+    rinv = pow(1 << (64 * nl), -1, p)
+    X, Y, Z = (sum(int(v) << (64 * i) for i, v in enumerate(jac[k * nl:(k + 1) * nl])) * rinv % p for k in range(3))
+    xy = [0, 0]
+    if Z:
+        zi = pow(Z, -1, p)
+        xy = [X * zi * zi % p, Y * zi * zi * zi % p]
+    limbs = np.array([[(v >> (64 * i)) & 0xFFFFFFFFFFFFFFFF for i in range(nl)] for v in xy], dtype=np.uint64)
+    return words32(limbs)
+
+
+def dump_outputs(outdir, outputs):
+    """--dump-outputs: every array of `outputs` as outdir/<name>.npy.  All values are float64
+    holding integers below 2^53 exactly, so two builds can be compared array for array:
+      msm_bls12_381_affine   the headline MSM's group element (affine_words)
+      pallas_msm_affine      the Pallas MSM's group element
+      ntt_goldilocks         Goldilocks NTT output, (k, 2) 32-bit words, at the positions in
+      ntt_goldilocks_index   (all of them up to 2^20 points, else 2^20 drawn with seed 0)
+    The NTT transforms its buffer in place, so its array is the seeded input transformed
+    max(3, --warmup) + --steps times.  The NTT arrays are written by single-rank runs only: with
+    several ranks each holds a slab of a sharded transform."""
+    os.makedirs(outdir, exist_ok=True)
+    for name, a in outputs.items():
+        np.save(os.path.join(outdir, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 R_PALLAS = 0x40000000000000000000000000000000224698fc0994a8dd8c46eb2100000001   # order of the Pallas group
 
 
-def bench_pallas(args, torch, msm, parallel, barrier, max_over_ranks, rank, world):
+def bench_pallas(args, torch, msm, parallel, barrier, max_over_ranks, rank, world, outputs):
     """BASELINE.json config 4: Pallas MSM over 2^24 points, sharded by point-chunk over the ranks
     (2^21 points per GPU at N = 8), one all-gather of the 96-byte partial results + combine.
     Device-resident, strong scaling; checked by folding every rank's scalars onto the distinct
@@ -498,7 +553,7 @@ def bench_pallas(args, torch, msm, parallel, barrier, max_over_ranks, rank, worl
         for _ in range(max(3, args.warmup)):
             result = step()
         barrier()
-        iters = max(3, args.steps)
+        iters = args.steps
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(iters):
@@ -506,6 +561,7 @@ def bench_pallas(args, torch, msm, parallel, barrier, max_over_ranks, rank, worl
         e1.record()
         barrier()
         ms = max_over_ranks(e0.elapsed_time(e1) / iters)
+        outputs["pallas_msm_affine"] = affine_words(result, P_PALLAS, 4)
         folded = fold_scalars(sc, m, R_PALLAS)
         if world > 1:
             parts = parallel.all_gather_partials(folded.reshape(-1), "cuda").reshape(world * m, 4)
@@ -556,7 +612,7 @@ def bench_reference_gpu(args, torch, msm, ntt, _lib, pts_host, sc_host, ours_res
                 r_ = fn()
             return (time.perf_counter() - t0) / reps, r_
 
-        reps = max(1, min(2, args.steps))
+        reps = args.steps
         dt_ref_pin, r_ref = clock(lambda: ref_msm(pts_host, sc_host), reps)
         pts_pg, sc_pg = np.array(pts_host), np.array(sc_host)            # pageable copies (a Rust Vec is pageable)
         dt_ref_pg, _ = clock(lambda: ref_msm(pts_pg, sc_pg), reps)
@@ -593,7 +649,7 @@ def bench_reference_gpu(args, torch, msm, ntt, _lib, pts_host, sc_host, ours_res
                 d2 = d1.clone()
                 p1, p2 = d1.data_ptr(), d2.data_ptr()
 
-                def timed(fn, stream, iters=10):
+                def timed(fn, stream, iters=args.steps):
                     for _ in range(3):
                         fn()
                     torch.cuda.synchronize()
@@ -626,7 +682,7 @@ def bench_reference_gpu(args, torch, msm, ntt, _lib, pts_host, sc_host, ours_res
         pin[:] = np.random.default_rng(9).integers(0, GL_P, size=nn, dtype=np.uint64)
         pg = np.array(pin)
 
-        def host_ms(fn, buf, reps=3):
+        def host_ms(fn, buf, reps=args.steps):
             fn(buf)
             t0 = time.perf_counter()
             for _ in range(reps):
@@ -652,7 +708,7 @@ def bench_reference_gpu(args, torch, msm, ntt, _lib, pts_host, sc_host, ours_res
 def bench_polynomial(args, torch, _lib, refdir):
     """SURVEY.md section 8 row f4 next to the reference's own polynomial/ kernels (oracle/ref_poly.cu
     built for sm_100a): Goldilocks, 2^lg_ntt elements resident in HBM (128 MiB at 2^24, larger
-    than L2), CUDA events on the stream each side launches on, mean of 10 calls back to back."""
+    than L2), CUDA events on the stream each side launches on, mean of --steps calls back to back."""
     path = os.path.join(refdir, "libref_poly_gl64_gpu.so")
     if not os.path.exists(path):
         raise FileNotFoundError(path)
@@ -671,7 +727,7 @@ def bench_polynomial(args, torch, _lib, refdir):
     cur, rs = torch.cuda.current_stream(), torch.cuda.ExternalStream(ref.ref_poly_stream())
     s = cur.cuda_stream
 
-    def timed(fn, stream, iters=10):
+    def timed(fn, stream, iters=args.steps):
         for _ in range(3):
             fn()
         stream.synchronize()
@@ -708,7 +764,7 @@ def bench_polynomial(args, torch, _lib, refdir):
     return {"workload": f"Goldilocks, 2^{args.lg_ntt} elements, device resident", **rows}
 
 
-def bench_ntt(args, torch, ntt, _lib, peak, peak_src, barrier, max_over_ranks, world):
+def bench_ntt(args, torch, ntt, _lib, peak, peak_src, barrier, max_over_ranks, world, outputs):
     """Goldilocks 2^lg NTT, NN order, device-resident (NTT::Base_dev_ptr path) and e2e
     (compute_ntt with a pinned host buffer).  With N > 1 ranks ONE transform is slab-sharded over
     the ranks (column slabs, one NCCL all-to-all between the two local passes; strong scaling)."""
@@ -722,7 +778,7 @@ def bench_ntt(args, torch, ntt, _lib, peak, peak_src, barrier, max_over_ranks, w
     host[:] = rng.integers(0, GL_P, size=n, dtype=np.uint64)
     d = host_t.cuda()
     flush = torch.empty(256 << 20, dtype=torch.uint8, device="cuda")
-    iters = max(10, args.steps * 5)
+    iters = args.steps
     for _ in range(max(3, args.warmup)):
         ntt.ntt_dev(d, ntt.NN)
     barrier()
@@ -736,6 +792,11 @@ def bench_ntt(args, torch, ntt, _lib, peak, peak_src, barrier, max_over_ranks, w
         e1.synchronize()
         tot += e0.elapsed_time(e1)
     ms = max_over_ranks(tot / iters)
+    if args.dump_outputs:            # d holds the last timed transform's output until the profiled one below
+        idx = np.arange(n) if n <= NTT_DUMP_SAMPLE else \
+            np.sort(np.random.default_rng(0).choice(n, NTT_DUMP_SAMPLE, replace=False))
+        outputs["ntt_goldilocks_index"] = idx
+        outputs["ntt_goldilocks"] = words32(d[torch.from_numpy(idx).cuda()].cpu().numpy().view(np.uint64)[:, None])
     _lib.profile_enable(True)
     flush.zero_()
     ntt.ntt_dev(d, ntt.NN)
@@ -764,7 +825,7 @@ def bench_ntt(args, torch, ntt, _lib, peak, peak_src, barrier, max_over_ranks, w
     # e2e: in place on the pinned host buffer through compute_ntt
     ntt.NTT(0 if world == 1 else torch.cuda.current_device(), host, ntt.NN)
     t0 = time.perf_counter()
-    reps = 5
+    reps = args.steps
     for _ in range(reps):
         ntt.NTT(0 if world == 1 else torch.cuda.current_device(), host, ntt.NN)
     dt = (time.perf_counter() - t0) / reps
@@ -845,8 +906,8 @@ def bench_ntt_sharded(args, torch, _lib, peak, peak_src, barrier, max_over_ranks
                              "frac": alg / (ms * 1e-3) / 1e9 / (peak * world), "traffic": None, "peak_source": peak_src},
                 "e2e": None}
 
-    res = run(0, args.lg_ntt, "Goldilocks", 8, max(10, args.steps * 5))
-    res["babybear_2pow27"] = run(1, 27, "BabyBear", 4, max(5, args.steps * 2))
+    res = run(0, args.lg_ntt, "Goldilocks", 8, args.steps)
+    res["babybear_2pow27"] = run(1, 27, "BabyBear", 4, args.steps)
     return res
 
 

@@ -178,6 +178,29 @@ def lde(field, evals, lg_blowup):
     return fn(ext, NN, False, True), c
 
 
+def ntt256_inputs():
+    """{lg: input} of the 256-bit NTT recording (tests/golden/make_golden.py ntt256), lg 1..10:
+    BLS12-381 scalar-field residues, (2^lg, 4) uint64, drawn in turn from random.Random(11)."""
+    import random
+    r = 0x73eda753299d7d483339d80809a1d80553bda402fffe5bfeffffffff00000001
+    rnd = random.Random(11)
+    return {lg: np.array([int_to_limbs(rnd.randrange(r), 4) for _ in range(1 << lg)], dtype=np.uint64)
+            for lg in range(1, 11)}
+
+
+def ntt256_golden(path):
+    """tests/golden/ntt256_ref_gpu.npz as a dict of every in_<lg> and
+    out_<lg>_<order><direction><type>.  Two kinds of array are not stored: the inputs, which are
+    ntt256_inputs(), and the RR outputs of the plain (non-coset) transforms, which the reference
+    computes bit for bit equal to the NN ones (the file stays below 1 MB)."""
+    g = dict(np.load(path))
+    for lg, x in ntt256_inputs().items():
+        g[f"in_{lg}"] = x
+        for d in range(2):
+            g[f"out_{lg}_3{d}0"] = g[f"out_{lg}_0{d}0"]
+    return g
+
+
 # ---------------------------------------------------------------- BLS12-381 G2 (oracle/ec2.c)
 def fp2_op(op, a, b=None):
     """Element-wise Fp2 op on (n, 12) Montgomery limb arrays: mul, add, sub, sqr, inv."""

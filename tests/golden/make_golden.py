@@ -13,8 +13,12 @@
                     `... make_golden.py g2_bn254|g2_bls12_377`.
   poly_<field>_ref_gpu.npz  the reference's polynomial/ templates (prefix_op, div_by_x_minus_z,
                     evaluate) through oracle/ref_poly.cu: `... make_golden.py poly_gl64|poly_bb31|poly_bls12_381_fr`.
-  msm_ref_cpu.npz   the reference's CPU msm/pippenger.hpp (oracle/_ref/libref_msm_cpu.so);
-                    runs anywhere: `python tests/golden/make_golden.py cpu`.
+  msm_ref_cpu.npz, msm_ref_cpu_n700.npz   the reference's CPU msm/pippenger.hpp
+                    (oracle/_ref/libref_msm_cpu.so); runs anywhere: `python tests/golden/make_golden.py cpu`.
+  msm_ref_gpu_2pow26.npz  the reference's CUDA mult_pippenger on the 2^26-point input of
+                    tests/test_msm_gpu.py: `... make_golden.py msm_2pow26` on a GPU.
+  ref_params.json   the parameter tables of the reference's headers, read from a checkout of it:
+                    `python tests/golden/make_golden.py params <reference checkout>`.
 
 tests/test_oracle.py checks the CPU oracle against all three, which is what pins it.
 Inputs are seeded; nothing here reads /root/reference at run time (only the prebuilt _ref .so).
@@ -74,6 +78,15 @@ def gen_cpu(outdir):
         out[f"affine_{n}"] = o.jac_to_affine("bls12_381", jac)
     np.savez_compressed(os.path.join(outdir, "msm_ref_cpu.npz"), **out)
     print("wrote msm_ref_cpu.npz")
+    # 700 points: 50 distinct multiples of G, scalars uniform below r (random.Random(3))
+    import random
+    rnd = random.Random(3)
+    n = 700
+    pts = o.gen_points("bls12_381", 50)[np.arange(n) % 50].copy()
+    sc = np.array([o.int_to_limbs(rnd.randrange(R_BLS), 4) for _ in range(n)], dtype=np.uint64)
+    affine = o.jac_to_affine("bls12_381", o.ref_cpu_msm(pts, sc, nthreads=4))
+    np.savez_compressed(os.path.join(outdir, "msm_ref_cpu_n700.npz"), pts=pts, sc=sc, affine=affine)
+    print("wrote msm_ref_cpu_n700.npz")
 
 
 # Every reference library is loaded in a process of its own: the reference's NTT keeps its
@@ -125,12 +138,8 @@ def gen_ntt256(outdir):
     lib = C.CDLL(o.ref_path("libref_ntt_bls12_381_gpu.so"))
     lib.compute_ntt.restype = RE
     lib.compute_ntt.argtypes = [C.c_size_t, C.c_void_p, C.c_uint32, C.c_int, C.c_int, C.c_int]
-    import random
-    rnd = random.Random(11)
     out = {}
-    for lg in range(1, 11):
-        x = np.array([o.int_to_limbs(rnd.randrange(R_BLS), 4) for _ in range(1 << lg)], dtype=np.uint64)
-        out[f"in_{lg}"] = x
+    for lg, x in o.ntt256_inputs().items():
         for order in range(4):
             for direction in range(2):
                 for typ in range(2):
@@ -138,6 +147,10 @@ def gen_ntt256(outdir):
                     e = lib.compute_ntt(0, y.ctypes.data, lg, order, direction, typ)
                     assert e.code == 0
                     out[f"out_{lg}_{order}{direction}{typ}"] = y
+        # not stored, restored by oracle.pyoracle.ntt256_golden: the input (ntt256_inputs) and the
+        # RR outputs of the plain transforms, equal to the NN ones
+        for direction in range(2):
+            assert np.array_equal(out.pop(f"out_{lg}_3{direction}0"), out[f"out_{lg}_0{direction}0"])
     np.savez_compressed(os.path.join(outdir, "ntt256_ref_gpu.npz"), **out)
     print("wrote ntt256_ref_gpu.npz")
 
@@ -156,6 +169,27 @@ def gen_msm(outdir):
         out[f"affine_{n}"] = o.jac_to_affine("bls12_381", jac)
     np.savez_compressed(os.path.join(outdir, "msm_ref_gpu.npz"), **out)
     print("wrote msm_ref_gpu.npz")
+
+
+def gen_msm_2pow26(outdir):
+    """msm_ref_gpu_2pow26.npz: the reference's CUDA mult_pippenger on 2^26 points, the 2^16
+    multiples (i+1)*G replicated, scalars uniform below 2^254 from default_rng(26) in blocks of
+    2^22 rows -- the input of tests/test_msm_gpu.py::test_bls12_381_msm_2pow26_equals_reference_gpu."""
+    lib = C.CDLL(o.ref_path("libref_msm_gpu.so"))
+    lib.mult_pippenger.restype = RE
+    lib.mult_pippenger.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]
+    n, m = 1 << 26, 1 << 16
+    pts = np.empty((n, 12), dtype=np.uint64)
+    pts.reshape(n // m, m, 12)[:] = o.gen_points("bls12_381", m)
+    rng = np.random.default_rng(26)
+    sc = np.empty((n, 4), dtype=np.uint64)
+    for s in range(0, n, 1 << 22):
+        sc[s:s + (1 << 22)] = rng.integers(0, 2**64, size=(1 << 22, 4), dtype=np.uint64)
+    sc[:, 3] >>= np.uint64(2)
+    jac = np.zeros(18, dtype=np.uint64)
+    ok(lib.mult_pippenger(jac.ctypes.data, pts.ctypes.data, n, sc.ctypes.data), "mult_pippenger 2^26")
+    np.savez_compressed(os.path.join(outdir, "msm_ref_gpu_2pow26.npz"), out=jac)
+    print("wrote msm_ref_gpu_2pow26.npz")
 
 
 def gen_gpu(outdir):
@@ -375,6 +409,66 @@ def gen_poly(outdir, field):
     print(f"wrote poly_{field}_ref_gpu.npz")
 
 
+def gen_params(outdir, ref):
+    """ref_params.json: the parameter tables the reference hard-codes in its headers (roots of
+    unity, domain-size inverses, Montgomery constants), read from the reference checkout `ref`,
+    as hex strings (tests/test_params_pin.py compares the derived values with them)."""
+    import json
+    import re
+
+    def small_table(path, name):
+        s = open(path).read()
+        tail = s.split("#endif")[-1]
+        if "#else" in s:
+            s = s.split("#else")[1].split("#endif")[0]
+        m = re.search(r"const fr_t %s\[S \+ 1\] = \{(.*?)\};" % name, s + tail, re.S)
+        return [int(x, 16) for x in re.findall(r"fr_t\((0x[0-9a-f]+)u?\)", m.group(1))]
+
+    def words(path, name):
+        """32-bit words of a device-side constant of ff/*.hpp"""
+        s = open(path).read().split("namespace device")[1]
+        m = re.search(r"%s\[\d+\] = \{(.*?)\};" % name, s, re.S)
+        w = []
+        for v in re.findall(r"TO_CUDA_T\((0x[0-9a-f]+)\)", m.group(1)):
+            v = int(v, 16)
+            w += [v & 0xFFFFFFFF, v >> 32]
+        if not w:                                       # pasta.hpp lists plain 32-bit words
+            w = [int(v, 16) for v in re.findall(r"0x[0-9a-f]{8}", m.group(1))]
+        return w
+
+    def wide_tables(path):
+        s = open(path).read()
+        t = {}
+        for m in re.finditer(r"const fr_t (\w+)\[S \+ 1\] = \{(.*?)\};", s, re.S):
+            vals = []
+            for mm in re.finditer(r"FR_T\(vec256,(.*?)\)", m.group(2)):
+                l = [int(x.strip().rstrip("u"), 16) for x in mm.group(1).split(",")]
+                vals.append(sum(v << (64 * i) for i, v in enumerate(l)))
+            t[m.group(1)] = vals
+        m = re.search(r"const fr_t group_gen = FR_T\(vec256,(.*?)\)", s)
+        l = [int(x.strip().rstrip("u"), 16) for x in m.group(1).split(",")]
+        t["group_gen"] = [sum(v << (64 * i) for i, v in enumerate(l))]
+        return {k: t[k] for k in ("group_gen", "forward_roots_of_unity", "domain_size_inverse")}
+
+    out = {"ntt": {}, "ff": {}, "ntt256": {}}
+    for name in ("goldilocks", "baby_bear"):
+        out["ntt"][name] = {t: small_table(f"{ref}/ntt/parameters/{name}.h", t)
+                            for t in ("forward_roots_of_unity", "inverse_roots_of_unity", "domain_size_inverse")}
+    for hdr, names in (("bls12-381", ("BLS12_381_P", "BLS12_381_RR", "BLS12_381_one", "BLS12_381_r", "BLS12_381_rone")),
+                       ("pasta", ("Pallas_P", "Pallas_RR", "Pallas_one", "Vesta_P", "Vesta_RR", "Vesta_one")),
+                       ("alt_bn128", ("ALT_BN128_P", "ALT_BN128_RR", "ALT_BN128_one", "ALT_BN128_r", "ALT_BN128_rRR",
+                                      "ALT_BN128_rone")),
+                       ("bls12-377", ("BLS12_377_P", "BLS12_377_RR", "BLS12_377_one", "BLS12_377_r", "BLS12_377_rone"))):
+        out["ff"][hdr] = {n: words(f"{ref}/ff/{hdr}.hpp", n) for n in names}
+    for name in ("bls12_381", "vesta", "pallas", "alt_bn128", "bls12_377"):
+        out["ntt256"][name] = wide_tables(f"{ref}/ntt/parameters/{name}.h")
+    hexed = {sec: {k: {t: [hex(v) for v in vs] for t, vs in d.items()} for k, d in tab.items()} for sec, tab in out.items()}
+    with open(os.path.join(outdir, "ref_params.json"), "w") as f:
+        json.dump(hexed, f, indent=1)
+        f.write("\n")
+    print("wrote ref_params.json")
+
+
 def gen_g2_curve(outdir, name):
     """msm_g2_<curve>_ref_gpu.npz: the reference's CUDA MSM templates over Fp2 for the msm crate's
     bn254 / bls12_377 features (oracle/ref_msm_g2.cu built with FEATURE_BN254 / FEATURE_BLS12_377:
@@ -412,6 +506,8 @@ if __name__ == "__main__":
     mode = sys.argv[1] if len(sys.argv) > 1 else "cpu"
     if mode == "cpu":
         gen_cpu(HERE)
+    elif mode == "params":
+        gen_params(HERE, sys.argv[2])
     else:
         outdir = os.path.join(ROOT, "gpurun_out", "golden")
         os.makedirs(outdir, exist_ok=True)
@@ -429,6 +525,8 @@ if __name__ == "__main__":
             gen_ntt256(outdir)
         elif mode == "msm":
             gen_msm(outdir)
+        elif mode == "msm_2pow26":
+            gen_msm_2pow26(outdir)
         elif mode in ("g2_bn254", "g2_bls12_377"):
             gen_g2_curve(outdir, mode[3:])
         elif mode.startswith("poly_"):

@@ -57,7 +57,7 @@ def test_reference_poc_glue_compiles_unmodified(lib):
     they lie, with plain g++ and -I include/compat: the reference's C++ callers switch libraries by
     switching the include path."""
     if not os.path.isdir("/root/reference"):
-        pytest.skip("reference sources are not on this machine")
+        pytest.skip("needs a checkout of the original project: its poc glue sources cannot be part of this repository")
     built = _builder().build_reference_glue()
     assert len(built) == 7
     syms = subprocess.check_output(["nm", "-D", os.path.join(OUT, "libdropin_msm.so")], text=True)
@@ -140,7 +140,7 @@ def test_reference_poc_glue_runs_on_this_library(oracle):
     against include/compat, shipped as tests/cpp/_build/libdropin_*.so) give the oracle's answers."""
     path = os.path.join(OUT, "libdropin_msm.so")
     if not os.path.exists(path):
-        pytest.skip("glue libraries were not built (no reference sources on the build machine)")
+        pytest.skip("needs the glue libraries built from the original project's poc sources, which cannot be part of this repository")
     glue = C.CDLL(path)
     for f in (glue.mult_pippenger_inf, glue.mult_pippenger_fp2_inf):
         f.restype, f.argtypes = RE, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t]

@@ -194,7 +194,8 @@ def test_ntt_256bit_matches_reference_gpu_golden():
     the reference's own 256-bit ("wide") CUDA kernels."""
     import os
     from sppark_b200 import ntt
-    g = np.load(os.path.join(os.path.dirname(__file__), "golden", "ntt256_ref_gpu.npz"))
+    from oracle import pyoracle
+    g = pyoracle.ntt256_golden(os.path.join(os.path.dirname(__file__), "golden", "ntt256_ref_gpu.npz"))
     for lg in range(1, 11):
         x = g[f"in_{lg}"]
         for order in range(4):
